@@ -2,6 +2,7 @@
 """Benchmark of the hot path: pyredner.RenderFunction forward + backward == two redner.render() calls.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|c3|c4|c5] [--mode tiles|poses|both]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 Workloads (BASELINE.json configs, SURVEY.md section 8d; meshes of C3 - C5 are the reference's own, tests/golden/scene_*.npz):
@@ -21,6 +22,11 @@ One "step" = one forward render + one backward render == W*H*spp pixel samples t
          the image, the loss and all gradients are inside the timed region;
   roofline      dominant kernel / stage of the step: algorithmic bytes of SURVEY.md section 8(d) over its CUDA-event duration;
   cpu_baseline  the unmodified reference (oracle/_ref, CPU/Embree) on a bounded sample of the same workload (rank 0, N = 1 only).
+
+--dump-outputs DIR: after the timed steps, rank 0 writes what the last timed step computed -- the image(s) of the forward call
+(`image`, poses stacked along a leading axis when a rank renders several) and every gradient the backward call returns (`grad<i>`, i =
+position in RenderFunction.backward's output, after the gradient all-reduce) -- as DIR/<name>.npy in float32.  Inputs are seeded, so two
+builds can be compared output for output.  Outputs larger than 64 MB in all are cut to a fixed, seeded sample of their elements.
 
 N > 1, one process per GPU.  `tiles` (the partition north_star names; the headline `value`): ONE image split into 4-row stripes
 round-robin over the ranks, all-reduce of framebuffer and gradients (strong scaling).  `poses`: every rank renders a full image
@@ -73,6 +79,26 @@ def timed_builds_ms(builds, n_timed):
     the memory pool (reported separately as scene_build_first_ms)."""
     tail = builds[-n_timed:] if n_timed > 0 else builds
     return sum(tail) / max(1, len(tail))
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Write {name: array} as out_dir/<name>.npy in float32.  If they exceed DUMP_BYTES in all, the small arrays are kept whole and
+    the larger ones are replaced by the same fixed, seeded sample of their flattened elements (distinct, sorted indices) on every
+    run, so that the files of two runs stay comparable element for element."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: np.ascontiguousarray(v, dtype=np.float32) for k, v in arrays.items()}
+    left, todo = DUMP_BYTES // 4, sorted(arrays, key=lambda k: arrays[k].size)
+    for i, name in enumerate(todo):
+        a = arrays[name]
+        take = min(a.size, left // (len(todo) - i))
+        if take < a.size:
+            a = a.ravel()[np.sort(np.random.RandomState(i).choice(a.size, take, replace=False))]
+        left -= a.size
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def measured_traffic(workload):
@@ -302,36 +328,45 @@ def run_ours(args, rank, world, local_rank):
             grads = api.RenderFunction.backward(ctx, d_img)
             ev[4].record()
             bwd_stats = c.scene.last_stage_stats()
-            tens = [g.to(dev, non_blocking=True) for g in grads if isinstance(g, torch.Tensor)]
-            return ev, tens, dict(build=c.scene.build_ms(), fwd_k=fwd_stats[0], bwd_k=bwd_stats[0], vertices=bwd_stats[1], hits=bwd_stats[2],
-                                  launches=c.scene.last_stats()[0])
+            tens = [(i, g.to(dev, non_blocking=True)) for i, g in enumerate(grads) if isinstance(g, torch.Tensor)]
+            return ev, img, tens, dict(build=c.scene.build_ms(), fwd_k=fwd_stats[0], bwd_k=bwd_stats[0], vertices=bwd_stats[1], hits=bwd_stats[2],
+                                       launches=c.scene.last_stats()[0])
 
         compute_ms = [0.0]
+        last = {}  # --dump-outputs: the images and gradients of the latest step
 
         def step():
-            total, acc, info = 0.0, None, None
+            total, acc, info, imgs = 0.0, None, None, []
             for sc in scs:
-                ev, tens, info = render_pair(sc)
-                acc = tens if acc is None else [a + b for a, b in zip(acc, tens)]
+                ev, img, tens, info = render_pair(sc)
+                grad_ids = [i for i, _ in tens]
+                acc = [g for _, g in tens] if acc is None else [a + b for a, (_, b) in zip(acc, tens)]
+                if args.dump_outputs:
+                    imgs.append(img)
                 e5 = ev[5]
                 if world > 1 and sc is scs[-1]:  # one packed gradient all-reduce per step (tiles: partial sums; poses: data parallel)
-                    rdist.all_reduce_packed(acc)
+                    acc = rdist.all_reduce_packed(acc)
                 e5.record()
                 torch.cuda.synchronize()
                 fwd, comm_f, bwd, comm_b = ev[0].elapsed_time(ev[1]), ev[1].elapsed_time(ev[2]), ev[3].elapsed_time(ev[4]), ev[4].elapsed_time(e5)
                 total += fwd + bwd + (comm_f + comm_b if world > 1 else 0.0)
                 compute_ms[0] += fwd + bwd
                 info.update(fwd_ms=fwd, bwd_ms=bwd, comm_ms=(comm_f + comm_b) if world > 1 else 0.0)
+            if args.dump_outputs:
+                last["image"] = imgs[0] if len(imgs) == 1 else torch.stack(imgs)
+                last.update(("grad%d" % i, g) for i, g in zip(grad_ids, acc))
             return total, info
-        return step, builds, compute_ms
+        return step, builds, compute_ms, last
 
     results = {}
     clocks = ClockSampler(local_rank)
     if rank == 0:
         clocks.start()
     for mode in modes:
-        step, builds, compute_ms = make_resident_step(mode)
+        step, builds, compute_ms, last = make_resident_step(mode)
         ms, rank_ms, infos = timed_loop(step, args.steps)
+        if args.dump_outputs and rank == 0 and mode == modes[0]:
+            dump_outputs(args.dump_outputs, {k: v.detach().cpu().numpy() for k, v in last.items()})
         imgs_per_step = (len(my_poses) if mode == "poses" else 1)
         job_imgs = (n_poses if n_poses else world) if mode == "poses" else 1
         per_rank, per_rank_compute = None, None
@@ -612,7 +647,12 @@ def main():
     ap.add_argument("--workload", default="c2", choices=sorted(WORKLOADS))
     ap.add_argument("--mode", default="both", choices=["both", "tiles", "poses"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's image and gradients to DIR/<name>.npy (float32); --impl ours only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank, world, local_rank = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1)), int(os.environ.get("LOCAL_RANK", 0))
     if args.impl == "reference":

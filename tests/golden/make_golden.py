@@ -23,7 +23,8 @@ sys.path.insert(0, os.path.join(ROOT, "tests"))
 import torch  # noqa: E402
 
 import ref_loader  # noqa: E402
-from parity_utils import CASES, GBUFFER_CASES, REFSTREAM_CASES, SCREEN_CASES, STAT_CASES, render_case, render_gbuffer, render_screen_gradient, render_stat_case  # noqa: E402
+from parity_utils import (CASES, CORNERS, GBUFFER_CASES, GPU_CASES, REFSTREAM_CASES, SCREEN_CASES, STAT_CASES, pixel_sample, render_case,  # noqa: E402
+                          render_corner, render_gbuffer, render_screen_gradient, render_stat_case)
 
 OUT = os.path.dirname(os.path.abspath(__file__))
 
@@ -72,6 +73,51 @@ def main():
                 arrs["samples." + k] = a
         np.savez_compressed(os.path.join(OUT, name + ".npz"), **arrs)
         print(name, {k: float(np.linalg.norm(v)) for k, v in arrs.items()})
+    for name, cfg in GPU_CASES.items():
+        if only and name not in only:
+            continue
+        img, grads = render_case(ref, dev, cfg, cfg["seed"], backward=name == "c2_shadow_blocker_128_sobol")
+        img = img.numpy()
+        arrs = {"pixels": img.reshape(-1, img.shape[-1])[pixel_sample(img.shape)], "image_max": np.float32(img.max())}
+        arrs.update({"grad." + k: v.numpy() for k, v in grads.items()})
+        np.savez_compressed(os.path.join(OUT, name + ".npz"), **arrs)
+        print(name, "image mean %.6f" % img.mean(), sorted(arrs))
+    for variant, chans, mb, edges, center in CORNERS:
+        name = "corner_ball_" + variant
+        if only and name not in only:
+            continue
+        img, grads = render_corner(ref, dev, variant, chans, mb, edges, center)
+        np.savez_compressed(os.path.join(OUT, name + ".npz"), image=img, **{"grad." + k: v.numpy() for k, v in grads.items()})
+        print(name, img.shape, sorted(grads))
+    if not only or "fuzz_reference" in only:
+        # the random scenes of tools/fuzz_emu.py that tests/test_device_code_cpu.py sweeps
+        sys.path.insert(0, os.path.join(ROOT, "tools"))
+        import fuzz_emu
+        fuzz_emu.save_reference(ref, os.path.join(OUT, "fuzz_reference.npz"), 0, 80)
+    if not only or "pyredner_envmap_tables" in only:
+        save_pyredner_envmap_tables(os.path.join(OUT, "pyredner_envmap_tables.npz"))
+
+
+def save_pyredner_envmap_tables(path):
+    """The sampling tables, pdf normalisation and mip pyramid the reference's Python layer builds for one seeded environment map
+    (pyredner/envmap.py, pyredner/texture.py), from the copy of pyredner that oracle/build_ref.sh places in oracle/_ref."""
+    import types
+    sys.path.insert(0, os.path.join(ROOT, "oracle", "_ref"))
+    for name in ("skimage", "skimage.io", "skimage.transform", "imageio"):  # (image I/O the envmap code does not use)
+        sys.modules.setdefault(name, types.ModuleType(name))
+    sys.modules["skimage"].io = sys.modules["skimage.io"]
+    sys.modules["skimage"].transform = sys.modules["skimage.transform"]
+    sys.modules["redner"] = ref_loader.load()
+    import pyredner
+    import parity_utils as pu
+    pyredner.set_use_gpu(False)
+    sky, e2w = pu.envmap_table_inputs()
+    a = pyredner.EnvironmentMap(sky, e2w)
+    arrs = {"sample_cdf_xs": a.sample_cdf_xs.numpy(), "sample_cdf_ys": a.sample_cdf_ys.numpy(), "pdf_norm": np.float64(a.pdf_norm),
+            "world_to_env": a.world_to_env.numpy()}
+    arrs.update({"mip%d" % i: m.detach().numpy() for i, m in enumerate(a.values.mipmap)})
+    np.savez_compressed(path, **arrs)
+    print(os.path.basename(path), sorted(arrs))
 
 
 if __name__ == "__main__":

@@ -294,3 +294,49 @@ def assert_screen_gradient_matches_golden(name, img):
     g = load_golden(name)["image"]
     assert img.shape == g.shape and np.linalg.norm(g) > 0
     assert rel_l2(img, g) < SCREEN_CASES[name]["tol"], rel_l2(img, g)
+
+
+# Larger configurations that only the GPU suite renders (tests/test_parity_gpu.py); the reference's outputs are stored under
+# the key's name.  Images larger than a few thousand pixels are stored as a fixed, seeded sample of PIXEL_SAMPLE pixels.
+GPU_CASES = {
+    "c2_shadow_blocker_128_sobol": dict(scene="shadow_blocker", res=128, spp=16, mb=1, sampler="sobol", edges=0, seed=11),
+    # 2000 intersecting random triangles (forward only)
+    "bvh_stress_random_soup": dict(scene="random_soup", res=128, spp=4, mb=2, sampler="sobol", edges=0, seed=4),
+    # the headline configuration itself, C2 at 512 x 512 x 64 spp (forward only)
+    "c2_full_size_forward_pixels": dict(scene="shadow_blocker", res=512, spp=64, mb=1, sampler="sobol", edges=0, seed=1),
+}
+PIXEL_SAMPLE = 4096
+
+
+def pixel_sample(shape, seed=0):
+    """Flat indices of the fixed pixel sample of an (H, W, C) image."""
+    return np.sort(np.random.RandomState(seed).choice(shape[0] * shape[1], PIXEL_SAMPLE, replace=False))
+
+
+def envmap_table_inputs():
+    """The seeded sky and rotation whose environment-map tables are stored as pyredner_envmap_tables.npz."""
+    g = torch.Generator().manual_seed(3)
+    sky = 0.1 + 2.0 * torch.rand(12, 24, 3, generator=g)
+    e2w = torch.tensor([[0.8, 0.0, 0.6, 0.0], [0.0, 1.0, 0.0, 0.0], [-0.6, 0.0, 0.8, 0.0], [0.0, 0.0, 0.0, 1.0]])
+    return sky, e2w
+
+
+CORNERS = [  # (variant, channels, max_bounces, primary edges, sample_pixel_center)
+    ("vcolor", ["radiance", "vertex_color", "diffuse_reflectance"], 1, True, False),
+    ("viewport", ["radiance"], 2, True, False),
+    ("plain", ["radiance", "uv", "shading_normal"], 1, False, True),
+    ("generic", ["radiance", "generic_texture"], 1, False, False),  # (the reference corrupts its heap with generic textures + edges)
+    ("invisible", ["radiance"], 3, True, False),
+]
+
+
+def render_corner(backend, device, variant, chans, mb, edges, center):
+    """scenes.corner_ball: image and every gradient of sum((img * w)^2), w weighting the channels differently."""
+    sc = scenes.corner_ball(device, variant=variant)
+    ch = [getattr(backend.channels, c) for c in chans]
+    args = api.RenderFunction.serialize_scene(sc, 4, mb, channels=ch, sampler_type=backend.SamplerType.sobol, device=device, backend=backend,
+                                              use_primary_edge_sampling=edges, use_secondary_edge_sampling=False, sample_pixel_center=center)
+    img = api.RenderFunction.apply(3, *args)
+    w = torch.linspace(0.5, 1.5, img.shape[-1], device=img.device)
+    (img * w).pow(2).sum().backward()
+    return img.detach().cpu().numpy(), collect_grads(sc)

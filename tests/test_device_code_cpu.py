@@ -91,10 +91,11 @@ def test_lean_instantiation_meets_the_goldens_it_serves(emulator_lean):
 
 def test_random_scene_sweep_against_the_live_reference(emulator):
     """tools/fuzz_emu.py on a fixed range of seeds: random cameras / meshes / materials / lamps / options rendered and
-    differentiated by the compiled reference and by the host build of the device headers; nothing may be flagged."""
-    if not os.path.isdir(os.path.join(ROOT, "oracle", "_ref")):
-        pytest.skip("oracle/_ref not built")
-    r = subprocess.run([sys.executable, "-W", "ignore", os.path.join(ROOT, "tools", "fuzz_emu.py"), emulator, "0", "80"], capture_output=True, text=True, timeout=900)
+    differentiated by the host build of the device headers and compared with the reference's outputs for the same scenes
+    (tests/golden/fuzz_reference.npz, written by tests/golden/make_golden.py); nothing may be flagged."""
+    golden = os.path.join(ROOT, "tests", "golden", "fuzz_reference.npz")
+    r = subprocess.run([sys.executable, "-W", "ignore", os.path.join(ROOT, "tools", "fuzz_emu.py"), emulator, "0", "80", "--golden", golden], capture_output=True,
+                       text=True, timeout=900)
     assert r.returncode == 0, r.stderr[-3000:]
     assert r.stdout.strip().splitlines()[-1] == "flagged 0 of 80", "\n".join(l for l in r.stdout.splitlines() if "<<<<" in l or "ERROR" in l)[-3000:]
 

@@ -1,5 +1,5 @@
-"""CPU suite, part 4: the drop-in claim.  Where the reference checkout is present (build container), the UNMODIFIED
-pyredner package is imported on top of redner_b200/dropin/redner.py and its own RenderFunction marshals a scene all the
+"""CPU suite, part 4: the drop-in claim.  Where oracle/build_ref.sh has placed the UNMODIFIED pyredner package in oracle/_ref, it
+is imported on top of redner_b200/dropin/redner.py and its own RenderFunction marshals a scene all the
 way into our C ABI (which then refuses to render without a GPU -- there is no CPU path)."""
 import os
 import subprocess
@@ -8,12 +8,12 @@ import sys
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
+REF = os.path.join(ROOT, "oracle", "_ref")  # the unmodified pyredner and the reference's native module (oracle/build_ref.sh)
 
 SCRIPT = r'''
 import sys, types
-sys.path.insert(0, %(dropin)r)
 sys.path.insert(0, %(ref)r)
+sys.path.insert(0, %(dropin)r)  # (ahead of the reference's own native `redner` module next to pyredner)
 for name in ("skimage", "skimage.io", "skimage.transform", "imageio"):
     sys.modules[name] = types.ModuleType(name)
 sys.modules["skimage"].io = sys.modules["skimage.io"]
@@ -39,7 +39,7 @@ except RuntimeError as e:
 '''
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "pyredner")), reason="reference checkout not present")
+@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "pyredner")), reason="oracle/_ref/pyredner not built")
 def test_unmodified_pyredner_runs_on_the_dropin_module():
     code = SCRIPT % {"dropin": os.path.join(ROOT, "redner_b200", "dropin"), "ref": REF}
     out = subprocess.run([sys.executable, "-W", "ignore", "-c", code], capture_output=True, text=True, timeout=300)
@@ -49,43 +49,25 @@ def test_unmodified_pyredner_runs_on_the_dropin_module():
     assert last.startswith("RENDERED") or ("ABI-ERROR" in last and "no CPU path" in last), last
 
 
-ENV_SCRIPT = r'''
-import sys, types
-sys.path.insert(0, %(dropin)r)
-sys.path.insert(0, %(ref)r)
-sys.path.insert(0, %(root)r)
-for name in ("skimage", "skimage.io", "skimage.transform", "imageio"):
-    sys.modules[name] = types.ModuleType(name)
-sys.modules["skimage"].io = sys.modules["skimage.io"]
-sys.modules["skimage"].transform = sys.modules["skimage.transform"]
-import torch, pyredner
-from redner_b200 import api
-g = torch.Generator().manual_seed(3)
-sky = 0.1 + 2.0 * torch.rand(12, 24, 3, generator=g)
-e2w = torch.tensor([[0.8, 0.0, 0.6, 0.0], [0.0, 1.0, 0.0, 0.0], [-0.6, 0.0, 0.8, 0.0], [0.0, 0.0, 0.0, 1.0]])
-pyredner.set_use_gpu(False)
-a = pyredner.EnvironmentMap(sky.clone(), e2w.clone())
-b = api.EnvironmentMap(sky.clone(), e2w.clone())
-assert torch.equal(a.sample_cdf_xs, b.sample_cdf_xs) and torch.equal(a.sample_cdf_ys, b.sample_cdf_ys), "sampling tables differ"
-assert abs(a.pdf_norm - b.pdf_norm) <= 1e-12 * abs(a.pdf_norm), (a.pdf_norm, b.pdf_norm)
-assert torch.equal(a.world_to_env, b.world_to_env)
-assert len(a.values.mipmap) == len(b.values.mipmap) and all(torch.allclose(x, y, atol=1e-7) for x, y in zip(a.values.mipmap, b.values.mipmap))
-print("ENVMAP-TABLES-OK")
-'''
-
-
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "pyredner")), reason="reference checkout not present")
 def test_envmap_preprocessing_matches_pyredner():
     """api.EnvironmentMap builds the importance-sampling tables, pdf normalisation and mip pyramid that the reference's Python
-    layer hands to the native EnvironmentMap (pyredner/envmap.py:36-61, pyredner/texture.py)."""
-    code = ENV_SCRIPT % {"dropin": os.path.join(ROOT, "redner_b200", "dropin"), "ref": REF, "root": ROOT}
-    out = subprocess.run([sys.executable, "-W", "ignore", "-c", code], capture_output=True, text=True, timeout=300)
-    assert out.returncode == 0 and "ENVMAP-TABLES-OK" in out.stdout, (out.stdout[-500:], out.stderr[-1500:])
+    layer hands to the native EnvironmentMap (pyredner/envmap.py:36-61, pyredner/texture.py); the reference's tables for the
+    same seeded map are stored in tests/golden/pyredner_envmap_tables.npz."""
+    import numpy as np
+    import torch
+    import parity_utils as pu
+    from redner_b200 import api
+    g = pu.load_golden("pyredner_envmap_tables")
+    sky, e2w = pu.envmap_table_inputs()
+    b = api.EnvironmentMap(sky, e2w)
+    assert np.array_equal(b.sample_cdf_xs.numpy(), g["sample_cdf_xs"]) and np.array_equal(b.sample_cdf_ys.numpy(), g["sample_cdf_ys"]), "sampling tables differ"
+    assert abs(g["pdf_norm"] - b.pdf_norm) <= 1e-12 * abs(g["pdf_norm"]), (g["pdf_norm"], b.pdf_norm)
+    assert np.array_equal(b.world_to_env.numpy(), g["world_to_env"])
+    mips = sorted((k for k in g if k.startswith("mip")), key=lambda k: int(k[3:]))
+    assert len(b.values.mipmap) == len(mips) and all(torch.allclose(x, torch.from_numpy(g[k]), atol=1e-7) for x, k in zip(b.values.mipmap, mips))
 
 
-
-
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "pyredner")), reason="reference checkout not present")
+@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "pyredner")), reason="oracle/_ref/pyredner not built")
 def test_unmodified_pyredner_gives_the_same_numbers_on_either_native_module(tmp_path):
     """The drop-in claim, numerically, without a GPU: the UNMODIFIED pyredner (its own serialize / unpack / forward / backward)
     renders and differentiates one scene twice -- on the reference's pybind module and on redner_b200/dropin/redner.py bound to
@@ -93,8 +75,6 @@ def test_unmodified_pyredner_gives_the_same_numbers_on_either_native_module(tmp_
     import numpy as np
     import test_device_code_cpu as tdc
     emu = tdc._build()
-    if not os.path.isdir(os.path.join(ROOT, "oracle", "_ref")):
-        pytest.skip("oracle/_ref not built")
     outs = {}
     for native in ("reference", emu):
         path = str(tmp_path / ("ref.npz" if native == "reference" else "ours.npz"))

@@ -1,7 +1,8 @@
 """CPU suite, part 3: host-side logic.
 
- * the host mirror of the pyredner interface (redner_b200/api.py) drives the UNMODIFIED reference module correctly:
-   argument marshalling, gradient-tuple alignment (one entry per serialized argument), seeds;
+ * the host mirror of the pyredner interface (redner_b200/api.py) drives a `redner` module correctly -- the UNMODIFIED reference
+   module where oracle/_ref is built, and the shim on the host build of the device headers: argument marshalling,
+   gradient-tuple alignment (one entry per serialized argument), seeds;
  * the `redner` shim marshals descriptors the way the reference's constructors read them;
  * the multi-GPU host logic (stripe partition, packed all-reduce, data-parallel pose loop) with the gloo backend and
    world_size 2.
@@ -21,22 +22,48 @@ from redner_b200 import api
 from redner_b200 import dist as rdist
 
 
-def test_backward_returns_one_gradient_per_argument(reference_module):
+@pytest.fixture
+def emu_backend(monkeypatch):
+    """The `redner` shim bound, for one test, to the host build of the device headers (tools/cpu_emu, test infrastructure)."""
+    import ctypes
+    import test_device_code_cpu as tdc
+    from redner_b200 import _lib, redner as rb
+    monkeypatch.setattr(_lib, "_lib", _lib._bind(ctypes.CDLL(tdc._build())))
+    return rb
+
+
+def _check_one_gradient_per_argument(backend):
     sc = scenes.glossy_room(torch.device("cpu"), resolution=(8, 8))
-    args = api.RenderFunction.serialize_scene(sc, 1, 1, device=torch.device("cpu"), backend=reference_module)
+    args = api.RenderFunction.serialize_scene(sc, 1, 1, device=torch.device("cpu"), backend=backend)
     img = api.RenderFunction.apply(3, *args)
     img.sum().backward()  # autograd itself checks len(grads) == len(inputs)
     assert sc.shapes[3].vertices.grad is not None and sc.area_lights[0].intensity.grad is not None
     assert sc.materials[0].diffuse_reflectance.texels.grad.shape == sc.materials[0].diffuse_reflectance.texels.shape
 
 
-def test_seed_convention(reference_module):
+def _check_seed_convention(backend):
     """backward seed = forward seed + 1000003 unless correlated random numbers are requested
     (pyredner/render_pytorch.py:658-663)."""
     sc = scenes.single_triangle(torch.device("cpu"), resolution=(8, 8))
-    args = api.RenderFunction.serialize_scene(sc, 1, 1, device=torch.device("cpu"), backend=reference_module)
+    args = api.RenderFunction.serialize_scene(sc, 1, 1, device=torch.device("cpu"), backend=backend)
     c = api.RenderFunction._unpack((5, 5 + 1000003), args)
     assert c.seed == (5, 1000008) and c.options.seed == 5
+
+
+def test_backward_returns_one_gradient_per_argument(emu_backend):
+    _check_one_gradient_per_argument(emu_backend)
+
+
+def test_backward_returns_one_gradient_per_argument_on_the_reference_module(reference_module):
+    _check_one_gradient_per_argument(reference_module)
+
+
+def test_seed_convention(emu_backend):
+    _check_seed_convention(emu_backend)
+
+
+def test_seed_convention_on_the_reference_module(reference_module):
+    _check_seed_convention(reference_module)
 
 
 def test_shim_marshalling_matches_reference_constructor_order():

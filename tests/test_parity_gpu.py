@@ -4,7 +4,7 @@
    (north_star tolerance; measured ~2e-7), sample-exact gradients within 1e-3 (measured ~1e-6 .. 1e-4);
  * secondary-edge (shadow) gradients, whose sample streams cannot be reproduced one-to-one: the mean over seeds must agree
    with the reference's mean within the combined standard error;
- * a live comparison with the compiled reference when oracle/_ref travelled with the snapshot;
+ * larger configurations and corner features against stored outputs of the reference (pu.GPU_CASES, pu.CORNERS);
  * size-independent properties at the full BASELINE size (512 x 512 x 64 spp): determinism, linearity in the emitted
    radiance, multi-GPU stripes == single image, gradient of a light intensity == image sum identity.
 """
@@ -116,51 +116,31 @@ def test_secondary_edge_gradients_statistically(rb, dev, name):
 
 
 def test_live_reference_if_present(rb, dev):
-    import ref_loader
-    if not ref_loader.available():
-        pytest.skip("oracle/_ref did not travel with this snapshot")
-    ref = ref_loader.load()
-    cfg = dict(scene="shadow_blocker", res=128, spp=16, mb=1, sampler="sobol", edges=0)
-    img_r, g_r = pu.render_case(ref, torch.device("cpu"), cfg, 11)
-    img_c, g_c = pu.render_case(rb, dev, cfg, 11)
-    assert pu.rel_l2(img_c.numpy(), img_r.numpy()) < IMG_TOL
-    for k in g_r:
-        assert pu.rel_l2(g_c[k].numpy(), g_r[k].numpy()) < GRAD_TOL, k
+    """C2 at 128 x 128 x 16 spp without edge sampling: image (fixed pixel sample) and every gradient against the reference's output."""
+    name = "c2_shadow_blocker_128_sobol"
+    cfg = pu.GPU_CASES[name]
+    g = pu.load_golden(name)
+    img_c, g_c = pu.render_case(rb, dev, cfg, cfg["seed"])
+    img_c = img_c.numpy()
+    assert pu.rel_l2(img_c.reshape(-1, img_c.shape[-1])[pu.pixel_sample(img_c.shape)], g["pixels"]) < IMG_TOL
+    assert set("grad." + k for k in g_c) == set(k for k in g if k.startswith("grad."))
+    for k in g_c:
+        assert pu.rel_l2(g_c[k].numpy(), g["grad." + k]) < GRAD_TOL, k
 
 
-CORNERS = [  # (variant, channels, max_bounces, primary edges, sample_pixel_center)
-    ("vcolor", ["radiance", "vertex_color", "diffuse_reflectance"], 1, True, False),
-    ("viewport", ["radiance"], 2, True, False),
-    ("plain", ["radiance", "uv", "shading_normal"], 1, False, True),
-    ("generic", ["radiance", "generic_texture"], 1, False, False),  # (the reference corrupts its heap with generic textures + edges)
-    ("invisible", ["radiance"], 3, True, False),
-]
-
-
-@pytest.mark.parametrize("variant,chans,mb,edges,center", CORNERS)
+@pytest.mark.parametrize("variant,chans,mb,edges,center", pu.CORNERS)
 def test_corner_features_against_live_reference(rb, dev, variant, chans, mb, edges, center):
     """Index buffers for uvs / normals, vertex colours, viewport crops, generic textures, pixel-centre sampling, invisible and
-    two-sided lights, deeper paths: image and every gradient against the compiled reference, where it travelled."""
-    import ref_loader
-    if not ref_loader.available():
-        pytest.skip("oracle/_ref did not travel with this snapshot")
-    ref = ref_loader.load()
-    out = []
-    for backend, device in ((ref, torch.device("cpu")), (rb, dev)):
-        sc = scenes.corner_ball(device, variant=variant)
-        ch = [getattr(backend.channels, c) for c in chans]
-        args = api.RenderFunction.serialize_scene(sc, 4, mb, channels=ch, sampler_type=backend.SamplerType.sobol, device=device, backend=backend,
-                                                  use_primary_edge_sampling=edges, use_secondary_edge_sampling=False, sample_pixel_center=center)
-        img = api.RenderFunction.apply(3, *args)
-        w = torch.linspace(0.5, 1.5, img.shape[-1], device=img.device)
-        (img * w).pow(2).sum().backward()
-        out.append((img.detach().cpu().numpy(), pu.collect_grads(sc)))
-    (img_r, g_r), (img_c, g_c) = out
+    two-sided lights, deeper paths: image and every gradient against the reference's output."""
+    img_c, g_c = pu.render_corner(rb, dev, variant, chans, mb, edges, center)
+    g = pu.load_golden("corner_ball_" + variant)
+    img_r = g["image"]
     assert img_r.shape == img_c.shape and pu.rel_l2(img_c, img_r) < IMG_TOL
-    assert set(g_r) == set(g_c)
-    for k in g_r:
-        if np.linalg.norm(g_r[k].numpy()) > 1e-9:
-            assert pu.rel_l2(g_c[k].numpy(), g_r[k].numpy()) < (5e-3 if edges and (k.endswith("vertices") or k.startswith("cam.")) else GRAD_TOL), k
+    assert set("grad." + k for k in g_c) == set(k for k in g if k.startswith("grad."))
+    for k in g_c:
+        r = g["grad." + k]
+        if np.linalg.norm(r) > 1e-9:
+            assert pu.rel_l2(g_c[k].numpy(), r) < (5e-3 if edges and (k.endswith("vertices") or k.startswith("cam.")) else GRAD_TOL), k
 
 
 def _render(rb, dev, res, spp, seed=1, intensity_scale=1.0, partition=None, edges=0, scene_fn=scenes.shadow_blocker):
@@ -200,19 +180,17 @@ def test_full_size_properties(rb, dev):
 
 
 def test_c2_full_size_forward_against_the_reference(rb, dev):
-    """The headline configuration itself, C2 at 512 x 512 x 64 spp (forward, fixed Sobol seed): relative L2 against the compiled
-    reference within north_star's 1e-4 where oracle/_ref travelled with the snapshot (the reference needs ~1 s for the forward
-    pass), and against the committed 8 x 8 block means of the reference's image in any case."""
-    cfg = dict(scene="shadow_blocker", res=512, spp=64, mb=1, sampler="sobol", edges=0)
-    img_c, _ = pu.render_case(rb, dev, cfg, 1, backward=False)
+    """The headline configuration itself, C2 at 512 x 512 x 64 spp (forward, fixed Sobol seed): relative L2 within north_star's 1e-4
+    against a fixed sample of the reference image's pixels and against its 8 x 8 block means."""
+    cfg = pu.GPU_CASES["c2_full_size_forward_pixels"]
+    img_c, _ = pu.render_case(rb, dev, cfg, cfg["seed"], backward=False)
     img_c = img_c.numpy()
     blocks = img_c.reshape(64, 8, 64, 8, 3).mean((1, 3))
     g = pu.load_golden("c2_full_size_forward_blocks")["blocks"]
     assert pu.rel_l2(blocks, g) < IMG_TOL, pu.rel_l2(blocks, g)
-    import ref_loader
-    if ref_loader.available():
-        img_r, _ = pu.render_case(ref_loader.load(), torch.device("cpu"), cfg, 1, backward=False)
-        assert pu.rel_l2(img_c, img_r.numpy()) < IMG_TOL, pu.rel_l2(img_c, img_r.numpy())
+    px = pu.load_golden("c2_full_size_forward_pixels")["pixels"]
+    mine = img_c.reshape(-1, 3)[pu.pixel_sample(img_c.shape)]
+    assert pu.rel_l2(mine, px) < IMG_TOL, pu.rel_l2(mine, px)
 
 
 def _translated_loss(rb, dev, scene, shape, shift, axis, res, spp, seed):
@@ -271,14 +249,12 @@ def test_ragged_and_degenerate_inputs(rb, dev):
 
 
 def test_bvh_stress_against_live_reference(rb, dev):
-    import ref_loader
-    if not ref_loader.available():
-        pytest.skip("oracle/_ref did not travel with this snapshot")
-    ref = ref_loader.load()
-    cfg = dict(scene="random_soup", res=128, spp=4, mb=2, sampler="sobol", edges=0)
-    img_r, _ = pu.render_case(ref, torch.device("cpu"), cfg, 4, backward=False)
-    img_c, _ = pu.render_case(rb, dev, cfg, 4, backward=False)
+    cfg = pu.GPU_CASES["bvh_stress_random_soup"]
+    img_c, _ = pu.render_case(rb, dev, cfg, cfg["seed"], backward=False)
+    img_c = img_c.numpy()
+    g = pu.load_golden("bvh_stress_random_soup")
+    px_c, px_r = img_c.reshape(-1, 3)[pu.pixel_sample(img_c.shape)], g["pixels"]
     # 2000 intersecting random triangles: a handful of silhouette samples may resolve differently in fp32
-    assert pu.rel_l2(img_c.numpy(), img_r.numpy()) < 5e-3
-    d = np.abs(img_c.numpy() - img_r.numpy()).max(-1)
-    assert (d > 1e-3 * img_r.numpy().max()).mean() < 2e-3
+    assert pu.rel_l2(px_c, px_r) < 5e-3
+    d = np.abs(px_c - px_r).max(-1)
+    assert (d > 1e-3 * g["image_max"]).mean() < 2e-3

@@ -2,12 +2,13 @@
 differentiated by (a) the compiled unmodified reference (oracle/_ref) and (b) the device headers compiled with g++
 (tools/cpu_emu), through the same host code; every image and gradient is compared.
 
-Development tool (needs /root/reference to have been compiled into oracle/_ref).  Combinations on which the reference
+The reference's outputs come from the compiled reference (oracle/_ref) or, with --golden, from a file written by
+save_reference (tests/golden/fuzz_reference.npz holds seeds 0 - 79).  Combinations on which the reference
 itself corrupts its heap are not generated (no radiance channel with bounces, generic texture with primary edges:
 DESIGN.md section 4); with secondary edge sampling (sample streams not reproducible one-to-one) or textured scenes under
 primary edge sampling (stale footprints in the reference) only the non-geometric gradients are compared.
 
-usage: python tools/fuzz_emu.py <emulator.so> <first seed> <count> [--verbose]
+usage: python tools/fuzz_emu.py <emulator.so> <first seed> <count> [--verbose] [--golden <reference outputs.npz>]
 """
 import ctypes
 import math
@@ -202,11 +203,58 @@ def run(backend, seed):
     return img.detach().numpy(), grads, cfg
 
 
+STORED_PIXELS = 128
+
+
+def stored_pixels(img, seed):
+    """The pixels of an (H, W, C) image that save_reference keeps: a fixed, seeded sample of STORED_PIXELS of them, as (n, C)."""
+    flat = img.reshape(-1, img.shape[-1])
+    n = flat.shape[0]
+    return flat[np.sort(np.random.RandomState(seed).choice(n, min(n, STORED_PIXELS), replace=False))]
+
+
+def save_reference(ref, path, first, count):
+    """The reference's image (stored_pixels) and gradients of seeds first .. first + count - 1 as float32, packed into one array (one
+    zip member per array would double the file): `names` ("<seed>/image", "<seed>/<gradient>"), `shapes` (flattened), `ndims`, `data`."""
+    names, arrays = [], []
+    for seed in range(first, first + count):
+        img, grads, _ = run(ref, seed)
+        names.append("%d/image" % seed)
+        arrays.append(stored_pixels(img, seed))
+        for k, v in grads.items():
+            names.append("%d/%s" % (seed, k))
+            arrays.append(v.numpy())
+    np.savez_compressed(path, names=np.array(names), ndims=np.array([a.ndim for a in arrays], dtype=np.int32),
+                        shapes=np.array([d for a in arrays for d in a.shape], dtype=np.int32),
+                        data=np.concatenate([a.astype(np.float32).ravel() for a in arrays]))
+
+
+def stored_reference(path, seed):
+    """Image pixels (stored_pixels) and gradients of one seed from a file written by save_reference."""
+    z = np.load(path)
+    shapes, data = z["shapes"], z["data"]
+    pre = "%d/" % seed
+    img, grads, dim, off = None, {}, 0, 0
+    for name, nd in zip(z["names"], z["ndims"]):
+        shape = tuple(int(d) for d in shapes[dim:dim + nd])
+        size = int(np.prod(shape))
+        if name.startswith(pre):
+            a = data[off:off + size].reshape(shape)
+            if name == pre + "image":
+                img = a
+            else:
+                grads[name[len(pre):]] = torch.from_numpy(a)
+        dim, off = dim + nd, off + size
+    return img, grads, make_case(seed)[1]
+
+
 def main():
     so, first, count = sys.argv[1], int(sys.argv[2]), int(sys.argv[3])
     verbose = "--verbose" in sys.argv
-    import ref_loader
-    ref = ref_loader.load()
+    golden = sys.argv[sys.argv.index("--golden") + 1] if "--golden" in sys.argv else None
+    if golden is None:
+        import ref_loader
+        ref = ref_loader.load()
     from redner_b200 import _lib
     _lib._lib = _lib._bind(ctypes.CDLL(so))
     from redner_b200 import redner as rb
@@ -217,13 +265,13 @@ def main():
     for seed in range(first, first + count):
         print("seed", seed, end=" ", flush=True)
         try:
-            ir, gr, cfg = run(ref, seed)
+            ir, gr, cfg = stored_reference(golden, seed) if golden else run(ref, seed)
             ic, gc, _ = run(rb, seed)
         except Exception as e:  # noqa: BLE001
             print("ERROR", type(e).__name__, str(e)[:200], flush=True)
             bad += 1
             continue
-        e_img = pu.rel_l2(ic, ir)
+        e_img = pu.rel_l2(stored_pixels(ic, seed) if golden else ic, ir)
         worst, wk = 0.0, "-"
         missing = set(gr) ^ set(gc)
         scale = max([float(np.linalg.norm(v.numpy())) for v in gr.values()], default=0.0)
